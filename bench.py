@@ -6,6 +6,7 @@
     torchrun --nproc-per-node N bench.py --gpus N ...              # one rank per GPU, batch sharded (weak scaling)
     python bench.py --config cfg3|cfg4|cfg5 ...                    # the other BASELINE.json workloads (see CONFIGS)
     python bench.py --scaling strong --gpus N                      # cfg2 with the GLOBAL batch of 64 split over N ranks
+    python bench.py --dump-outputs DIR ...                         # also write the last timed step's result as DIR/x_hat.npy
 
 cfg2 (the configuration the metric is quoted on): one "step" = one PnP-PGD iteration over the whole batch — fused L2 data
 step z = x - gamma (A^T A x - A^T y), then x = DRUNet(z, sigma) — through the package's public optimiser API
@@ -26,10 +27,12 @@ import tempfile
 import time
 from pathlib import Path
 
+import numpy as np
 import torch
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 
 SIGMA_DEN = 0.05
 STEPSIZE = 1.0
@@ -46,6 +49,22 @@ CONFIGS = {
              "H": 1024, "W": 1024, "metric": "pnp_admm_iterations_per_s", "unit": "it/s"},
 }
 REF_SAMPLE = 16  # images of the 64 the CPU arm runs per step
+DUMP_BYTES = 64 * 10 ** 6  # --dump-outputs budget over all arrays
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """`--dump-outputs`: each array as <out_dir>/<name>.npy in float32, so that two builds can be compared output for output.
+    An array larger than its share of DUMP_BYTES is replaced by a fixed seeded sample of its elements (flat, in index order):
+    the same positions on every run."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    cap = (DUMP_BYTES // len(arrays) - 4096) // 4  # elements per array (4096 bytes of room for the .npy header)
+    for name, t in arrays.items():
+        a = t.detach().float()
+        if a.numel() > cap:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            a = a.flatten()[idx.to(a.device)]
+        np.save(d / f"{name}.npy", a.cpu().numpy())
 
 
 def measured_peaks():
@@ -252,6 +271,8 @@ def run_reference(args):
     for _ in range(max(args.warmup, 0)):
         cpu_pgd_iteration_seconds(REF_SAMPLE, threads)
     ts = [cpu_pgd_iteration_seconds(REF_SAMPLE, threads) for _ in range(max(args.steps, 1))]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"x_hat": _cpu_state[REF_SAMPLE][3]})
     t = sum(ts) / len(ts)
     scale = c["batch"] / REF_SAMPLE
     value = 1.0 / (t * scale)  # every rank's shard is 64 images; at N GPUs the CPU host runs N shards one after another: N x work, N x time
@@ -523,6 +544,8 @@ def run_cfg2(args, world, rank, dev, peaks):
             torch.cuda.profiler.stop()
         ms_total = e0.elapsed_time(e1)
         x_hat = x_hat.clone()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"x_hat": gathered if gathered is not None else x_hat})
         launches = lib.dinvk_launch_count() - launches0
         if graphed is not None:
             launches = graphed.launches_per_step * args.steps
@@ -827,6 +850,7 @@ def timed_steps(step, steps, warmup, dev, world):
     if world > 1 and out is not None:
         gathered = torch.empty((world * out.shape[0], *out.shape[1:]), device=dev, dtype=out.dtype)
         dist.all_gather_into_tensor(gathered, out.contiguous())
+        out = gathered
     e1.record()
     torch.cuda.synchronize()
     t1 = ClockSampler.now()
@@ -908,6 +932,8 @@ def run_other(args, world, rank, dev, peaks):
 
         n0 = lib.dinvk_launch_count()
         ms_step, out, win = timed_steps(step, args.steps, args.warmup, dev, world)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"x_hat": out})
         launches = lib.dinvk_launch_count() - n0 - (0)
         launches = int(launches * args.steps / (args.steps + 0))
         ms_e2e = dist_max(time_cuda(e2e, max(2, min(args.steps, 5)), warmup=1), dev, world)
@@ -967,7 +993,11 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="time the eager Python loop instead of CUDA-graph replays")
     ap.add_argument("--verify-shards", action="store_true", help="strong scaling: compare the gathered result with rank 0 computing the whole batch")
     ap.add_argument("--lean", action="store_true", help="skip the rank-0 extras (parity, other precisions, rooflines, operators, CPU baseline)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the reconstruction of the last one as DIR/x_hat.npy "
+                                                          "(float32; a fixed seeded sample of it beyond 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

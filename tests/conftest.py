@@ -16,10 +16,14 @@ def pytest_configure(config):
 
 
 def load_golden(name: str) -> dict:
-    """npz fixture -> dict of torch tensors; keys `sd__a__b` are collected into a state_dict under 'sd'"""
-    z = np.load(GOLDEN / f"{name}.npz")
+    """npz fixture -> dict of torch tensors; keys `sd__a__b` are collected into a state_dict under 'sd'.  A fixture too large for
+    one file (every stored file stays under 1 MB) continues in golden/more/<name>.npz."""
+    z = dict(np.load(GOLDEN / f"{name}.npz"))
+    more = GOLDEN / "more" / f"{name}.npz"
+    if more.exists():
+        z.update(np.load(more))
     out, sd = {}, {}
-    for k in z.files:
+    for k in z:
         if k == "sd_from":  # the state_dict lives in another fixture (the seed-0 tiny DRUNet is shared by several cases)
             sd = dict(load_golden(str(z[k]))["sd"])
             continue

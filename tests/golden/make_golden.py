@@ -31,13 +31,28 @@ OUT = Path(__file__).resolve().parent
 assert dinv.__version__ == "0.4.1", dinv.__version__
 
 
+PART_BYTES = 800_000  # raw array bytes beyond which a fixture is split over two files: each stays under 1 MB compressed
+
+
 def save(name, **arrays):
     conv = {}
     for k, v in arrays.items():
         if isinstance(v, torch.Tensor):
             v = v.detach().cpu().numpy()
         conv[k] = np.asarray(v)
-    np.savez_compressed(OUT / f"{name}.npz", **conv)
+    parts = [{}, {}]
+    if sum(v.nbytes for v in conv.values()) > PART_BYTES:  # largest first, each into the lighter half; the second -> more/
+        for k in sorted(conv, key=lambda k: -conv[k].nbytes):
+            parts[sum(v.nbytes for v in parts[0].values()) > sum(v.nbytes for v in parts[1].values())][k] = conv[k]
+    else:
+        parts[0] = conv
+    np.savez_compressed(OUT / f"{name}.npz", **parts[0])
+    more = OUT / "more" / f"{name}.npz"
+    if parts[1]:
+        more.parent.mkdir(exist_ok=True)
+        np.savez_compressed(more, **parts[1])
+    else:
+        more.unlink(missing_ok=True)
     print(f"{name}: {len(conv)} arrays, {sum(v.nbytes for v in conv.values()) / 1024:.0f} KiB")
 
 
@@ -286,9 +301,11 @@ def sd_arrays(model, prefix):
     sd = model.state_dict()
     ref = OUT / "drunet_tiny.npz"
     if ref.exists():
-        base = np.load(ref)
+        base = dict(np.load(ref))
+        if (OUT / "more" / ref.name).exists():
+            base.update(np.load(OUT / "more" / ref.name))
         keys = {f"sd__{k.replace('.', '__')}" for k in sd}
-        if keys == {k for k in base.files if k.startswith("sd__")} and all(
+        if keys == {k for k in base if k.startswith("sd__")} and all(
                 np.array_equal(base[f"sd__{k.replace('.', '__')}"], v.numpy()) for k, v in sd.items()):
             return {"sd_from": np.array("drunet_tiny")}
     return {f"{prefix}{k.replace('.', '__')}": v for k, v in sd.items()}
@@ -563,15 +580,67 @@ def fastmri_fixture():
     save("fastmri_synth", **out)
 
 
+def callers_fixture():
+    """what the reference's own callers compute on the inputs of optim_mri_tiny / ddrm_mri_tiny / blur_gauss_circular_prox:
+    PGD / HQS, DDRM with a closed-form toy denoiser and the least-squares solvers (optim/linear) — the yardsticks of
+    tests/test_reference_callers_dropin.py"""
+    from deepinv.optim import HQS
+    from deepinv.optim.linear import least_squares
+
+    out = {}
+    o = np.load(OUT / "optim_mri_tiny.npz")
+    y, mask = torch.from_numpy(o["y"]), torch.from_numpy(o["mask"])
+    phys = MRI(mask=mask, img_size=(2, 32, 32))
+    toy = lambda v, s: v * (1.0 - float(s))
+    with torch.no_grad():
+        out["pgd"] = PGD(data_fidelity=L2(), prior=PnP(tiny_drunet(2)), stepsize=1.0, sigma_denoiser=0.05, max_iter=2,
+                         early_stop=False)(y, phys)
+        out["hqs_toy"] = HQS(data_fidelity=L2(), prior=PnP(toy), stepsize=0.8, sigma_denoiser=0.05, max_iter=3,
+                             early_stop=False)(y, phys)
+    d = np.load(OUT / "ddrm_mri_tiny.npz")
+    sig = float(d["sigma_noise"])
+    physd = MRI(mask=torch.from_numpy(d["mask"]), img_size=(2, 32, 32), noise_model=dinv.physics.GaussianNoise(sigma=sig))
+    it = iter(list(torch.from_numpy(d["noises"])))
+    orig = torch.randn_like
+    torch.randn_like = lambda t, **kw: next(it).to(t)
+    try:
+        out["ddrm_toy"] = dinv.sampling.DDRM(denoiser=lambda v, s: v * (1.0 / (1.0 + float(s))), sigmas=d["sigmas"])(
+            torch.from_numpy(d["y"]), physd)
+    finally:
+        torch.randn_like = orig
+    b = {k: torch.from_numpy(v) for k, v in np.load(OUT / "blur_gauss_circular_prox.npz").items()}
+    gam = float(b["gamma"])
+    circ, valid = Blur(filter=b["filt"], padding="circular"), Blur(filter=b["filt"], padding="valid")
+
+    def ls(p, y_, z, gamma, solver, max_iter, tol, normal=True):
+        kw = dict(AAT=p.A_A_adjoint, ATA=p.A_adjoint_A) if normal else {}
+        return least_squares(p.A, p.A_adjoint, y_, z=z, init=z, gamma=gamma, parallel_dim=[0], max_iter=max_iter, tol=tol,
+                             solver=solver, **kw)
+
+    yv = valid.A(b["z"])
+    out["valid_y"] = yv
+    for solver in ("CG", "BiCGStab"):
+        out[f"ls_{solver}"] = ls(circ, b["y"], b["z"], gam, solver, 25, 1e-5)
+    out["ls_valid_BiCGStab"] = ls(valid, yv, b["z"], gam, "BiCGStab", 25, 1e-5)
+    yl = valid.A(b["z"]) + 0.01 * torch.randn(valid.A(b["z"]).shape, generator=g(0))
+    out["lsqr_y"] = yl
+    out["lsqr_gamma2"] = ls(valid, yl, b["x"], 2.0, "lsqr", 30, 1e-6, normal=False)
+    out["lsqr_gamma_batched"] = ls(valid, yl, b["x"], torch.tensor([0.5, 3.0]), "lsqr", 30, 1e-6, normal=False)
+    out["minres_valid"] = ls(valid, yv, b["x"], 2.0, "minres", 30, 1e-6)
+    out["minres_circular"] = ls(circ, b["y"], b["z"], 2.0, "minres", 15, 1e-6)
+    save("reference_callers", **out)
+
+
 if __name__ == "__main__":
     torch.set_num_threads(8)
-    which = sys.argv[1:] or ["mri", "multicoil", "tomo", "blur", "blurfft", "model", "optim", "ddrm", "optim2", "train", "dynamic", "down", "combine", "maskgen", "mri3d", "fan", "anderson", "diffpir", "inpainting", "fastmri"]
+    which = sys.argv[1:] or ["mri", "multicoil", "tomo", "blur", "blurfft", "model", "optim", "ddrm", "optim2", "train", "dynamic", "down", "combine", "maskgen", "mri3d", "fan", "anderson", "diffpir", "inpainting", "fastmri", "callers"]
     table = {"mri": mri_fixtures, "multicoil": multicoil_fixtures, "tomo": tomo_fixtures, "blur": blur_fixtures,
              "blurfft": blurfft_fixtures, "model": model_fixtures, "optim": optim_fixtures, "ddrm": ddrm_fixture,
              "optim2": optim2_fixtures, "train": train_fixtures,
              "dynamic": dynamic_fixtures, "down": down_fixtures,
              "combine": combine_fixtures, "maskgen": maskgen_fixtures,
              "mri3d": mri3d_fixture, "fan": fanbeam_fixtures, "anderson": anderson_fixtures,
-             "diffpir": diffpir_fixture, "inpainting": inpainting_fixture, "fastmri": fastmri_fixture}
+             "diffpir": diffpir_fixture, "inpainting": inpainting_fixture, "fastmri": fastmri_fixture,
+             "callers": callers_fixture}
     for w in which:
         table[w]()
